@@ -149,6 +149,39 @@ def pose_sha(P):
     return hashlib.sha256(np.ascontiguousarray(np.asarray(P, dtype=np.float64)).tobytes()).hexdigest()
 
 
+LM_SUMMARY_FIELDS = ("termination", "num_iterations", "num_successful_steps", "num_evaluations", "num_linear_solves",
+                     "initial_cost", "final_cost")
+NN_SAMPLE_ROWS = 1_500_000   # 4 float64 columns: 48 MB, which keeps the whole dump under 64 MB
+NN_SAMPLE_SEED = 0xD0
+
+
+def dump_outputs(out_dir, eng, sc, edges, poses, summary, world):
+    """What the last timed step handed its caller, as .npy files in out_dir, so that two builds run with the same arguments can be
+    compared output for output: poses.npy (float64 [M, 4, 4]) and lm_summary.npy (float64, LM_SUMMARY_FIELDS in that order); with
+    one GPU, per edge edge_inliers.npy / edge_weights.npy (float64 / float32 [E]) and, for a fixed seeded sample of every free
+    frame's queries, nn_edge / nn_query / nn_idx / nn_d2.npy (float64 [rows]): the edge, the query point, its nearest neighbour in
+    the destination frame and their squared distance (every list in full would exceed 64 MB at configs 3-5)."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "poses.npy"), np.asarray(poses, np.float64))
+    np.save(os.path.join(out_dir, "lm_summary.npy"), np.array([summary[k] for k in LM_SUMMARY_FIELDS], np.float64))
+    if world > 1:     # a rank holds the correspondences of its own edges only
+        return
+    cw = [eng.get_edge(e, arrays=False) for e in range(len(edges))]
+    np.save(os.path.join(out_dir, "edge_inliers.npy"), np.array([c for c, _ in cw], np.float64))
+    np.save(os.path.join(out_dir, "edge_weights.npy"), np.array([w for _, w in cw], np.float32))
+    act = [e for e, (s, _) in enumerate(edges) if s != 0]
+    rng = np.random.default_rng(NN_SAMPLE_SEED)
+    cols = {"nn_edge": [], "nn_query": [], "nn_idx": [], "nn_d2": []}
+    for e in act:
+        n = len(sc["pts"][edges[e][0]])
+        q = np.sort(rng.choice(n, min(n, NN_SAMPLE_ROWS // len(act)), replace=False))
+        idx, d2 = eng.get_nn(e)
+        cols["nn_edge"].append(np.full(len(q), e, np.float64)); cols["nn_query"].append(q.astype(np.float64))
+        cols["nn_idx"].append(idx[q].astype(np.float64)); cols["nn_d2"].append(d2[q])
+    for k, v in cols.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.concatenate(v) if v else np.zeros(0))
+
+
 class ClockSampler(threading.Thread):
     """nvidia-smi clocks / throttle reasons during the timed region (profiling guide's clocks line)."""
 
@@ -398,13 +431,13 @@ def run_ours(args, cfg):
                 if mode == "mat":
                     en.correspond(CUTOFF)
                     nb = en.pull_all_edges()
-                    en.optimize(param, cost, True)
+                    s = en.optimize(param, cost, True)
                 else:
                     nb = 0
-                    en.icp_round(CUTOFF, param, cost, True)
+                    s = en.icp_round(CUTOFF, param, cost, True)
                 if mode != "dev":
                     poses = en.get_poses()     # device -> host
-                per.append(dict(d2h=nb))
+                per.append(dict(d2h=nb, summary=s))
             en.sync()
             return per, traj
         for r in range(k):
@@ -440,11 +473,13 @@ def run_ours(args, cfg):
     barrier()
     st0 = eng.stats(); l0 = st0["kernel_launches"]
     t0 = time.perf_counter()
-    run_rounds(eng, args.steps, "dev", stream, instrument=False)     # the timed K steps: nothing but the K calls
+    timed, _ = run_rounds(eng, args.steps, "dev", stream, instrument=False)     # the timed K steps: nothing but the K calls
     barrier()
     wall_total = time.perf_counter() - t0
     st1 = eng.stats(); l1 = st1["kernel_launches"]
     final_poses = eng.get_poses()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, sc, edges, final_poses, timed[-1]["summary"], world)
     # e2e: same K rounds, poses cross the C ABI as host buffers every step
     barrier()
     t0 = time.perf_counter()
@@ -616,7 +651,13 @@ def main():
     ap.add_argument("--single-rounds", type=int, default=2, help="reference arm: rounds of the single-thread leg (0: skip)")
     ap.add_argument("--check-cpu", action="store_true", help="replay every round on the CPU from the GPU's poses and compare counts / poses")
     ap.add_argument("--flags", type=int, default=0, help="MVICP_FLAG_* bits for the engine (A/B measurements)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy "
+                                                           "(poses, LM summary, per-edge counts / weights, a seeded sample of the NN answers)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         run_reference(args, cfg)

@@ -20,7 +20,14 @@ bunny18.npz      the reference's DEFAULT multiview workload (main_multiview.cpp:
                  (frame 0 = GT, the others addNoise(GT, 0.02, 0.01), common.h:38-67; the reference's default-seeded mt19937 stream
                  is not reproduced -- same noise model, numpy seed 0xB18).  Used by `bench.py --config real` and tests/test_gpu_real18.py.
 sophus_vectors.npz  the SE3 group elements / tangents of ext/sophus-ceres/test/core/test_se3.cpp:40-82 (values only).
+ref_pins.npz     answers of the reference's own code (oracle/_ref) that tests/test_oracle_corr.py and tests/test_oracle_functor_pin.py
+                 compare the oracle with, so that those comparisons run where the reference tree is absent:
+                 corr_*: nanoflann's 1-NN for edge 1 -> 0 of synth.make_scene(3, 20000, 32) under poses_init / poses_gt (every
+                 index, and the sha256 of the squared distances' bytes); knn_*: nanoflann's knnSearch(10) for every 53rd point of
+                 bunny_pair.npz's pts0; gfun_* / pfun_* / quat_*: inputs and outputs of the reference functor text for the first
+                 iterations of the seeded loops of test_oracle_functor_pin.py (a sample: the full loops would not fit in 1 MB).
 """
+import hashlib
 import os
 import sys
 
@@ -116,8 +123,66 @@ def sophus_vectors():
                         trans=np.array([e[1] for e in el], float), tangents=np.array(tg, float))
 
 
+def ref_pins():
+    import ctypes as C
+    sys.path.insert(0, os.path.dirname(OUT))
+    from test_oracle_functor_pin import _rand_pose
+    assert O.ref_lib() is not None and O.ref_functors() is not None, "oracle/_ref was not built"
+    out = {}
+    sc = synth.make_scene(3, 20000, config_id=32)
+    ref = O.KdIndex(sc["pts"][0], "ref")
+    for name in ("poses_init", "poses_gt"):
+        P = sc[name]
+        idx, d2 = ref.closest_points(sc["pts"][1], P[1], P[0], threads=4)
+        out[f"corr_{name}_idx"] = idx
+        out[f"corr_{name}_d2_sha256"] = np.array(hashlib.sha256(d2.tobytes()).hexdigest())
+    g = np.load(os.path.join(OUT, "bunny_pair.npz"))
+    pts = g["pts0"]
+    rf = O.KdIndex(pts, "ref")
+    q = np.arange(0, len(pts), 53)
+    res = [O.knn(rf, pts[i], 10) for i in q]
+    out["knn_query"] = q
+    out["knn_idx"] = np.stack([r[0] for r in res]); out["knn_d2"] = np.stack([r[1] for r in res])
+    for param in (0, 1, 2):
+        for plane in (0, 1):
+            G = 6 if param == 0 else 7
+            rng = np.random.default_rng(100 + 10 * param + plane)   # the loop of test_global_functors_match_reference_text
+            ins, rs, js = [], [], []
+            for it in range(32):
+                c1 = _rand_pose(rng, param, unit=it % 3 != 0); c2 = _rand_pose(rng, param, unit=it % 3 != 0)
+                if param == 0 and it % 50 == 0:
+                    c1[:3] = rng.normal(0, 1e-9, 3)
+                src = rng.normal(0, 0.3, 3); dst = rng.normal(0, 0.3, 3); nor = rng.normal(size=3); nor /= np.linalg.norm(nor)
+                r, j = O.functor_eval(param, plane, c1, c2, src, dst, nor, "ref")
+                ins.append(np.concatenate([c1, c2, src, dst, nor])); rs.append(r); js.append(j)
+            k = f"gfun_p{param}_l{plane}"
+            out[k + "_in"] = np.stack(ins); out[k + "_r"] = np.stack(rs); out[k + "_j"] = np.stack(js)
+            rng = np.random.default_rng(200 + 10 * param + plane)   # the loop of test_pairwise_functors_are_the_global_ones_with_identity_dst
+            ins, rs, js = [], [], []
+            for it in range(16):
+                c1 = _rand_pose(rng, param)
+                src = rng.normal(0, 0.3, 3); dst = rng.normal(0, 0.3, 3); nor = rng.normal(size=3); nor /= np.linalg.norm(nor)
+                r, j = O.functor_eval_pairwise_ref(param, plane, c1, src, dst, nor)
+                ins.append(np.concatenate([c1, src, dst, nor])); rs.append(r); js.append(j)
+            k = f"pfun_p{param}_l{plane}"
+            out[k + "_in"] = np.stack(ins); out[k + "_r"] = np.stack(rs); out[k + "_j"] = np.stack(js)
+    lib = O.ref_functors()
+    P = lambda a: a.ctypes.data_as(C.POINTER(C.c_double))
+    rng = np.random.default_rng(7)   # the loop of test_quaternion_parameterisation_matches_reference_text
+    xs, ds, pl, jac = [], [], [], []
+    for it in range(40):
+        x = rng.normal(size=4); x /= np.linalg.norm(x)
+        d = rng.normal(0, 0.3, 3) if it % 10 else np.zeros(3)
+        o = np.zeros(4); lib.ref_quat_plus(P(x), P(d), P(o))
+        j = np.zeros(12); lib.ref_quat_jacobian(P(x), P(j))
+        xs.append(x); ds.append(d); pl.append(o); jac.append(j)
+    out.update(quat_x=np.stack(xs), quat_d=np.stack(ds), quat_plus=np.stack(pl), quat_jac=np.stack(jac))
+    np.savez_compressed(os.path.join(OUT, "ref_pins.npz"), **out)
+    print("ref_pins:", os.path.getsize(os.path.join(OUT, "ref_pins.npz")) / 1e3, "kB")
+
+
 if __name__ == "__main__":
     only = sys.argv[1:]
-    for fn in (bunny_pair, dino_pair, lm_golden, sophus_vectors, bunny18):
+    for fn in (bunny_pair, dino_pair, lm_golden, sophus_vectors, bunny18, ref_pins):
         if not only or fn.__name__ in only:
             fn()

@@ -1,7 +1,9 @@
-"""Pins the oracle's correspondence restatement (oracle_icp.cpp) against the reference's own nanoflann compiled from
-/root/reference (oracle/_ref), against brute force, and against the committed golden vectors."""
+"""Pins the oracle's correspondence restatement (oracle_icp.cpp) against the reference's own nanoflann (its stored answers in
+tests/golden/ref_pins.npz, and the library itself when oracle/_ref was built), against brute force, and against the committed
+golden vectors."""
+import hashlib
+
 import numpy as np
-import pytest
 
 from helpers import scene
 from mv_lm_icp_b200 import synth
@@ -20,10 +22,16 @@ def test_kd_restatement_equals_brute_force(oracle):
         assert np.array_equal(a[0], b[0]) and np.array_equal(a[1].view(np.uint64), b[1].view(np.uint64))
 
 
-def test_restatement_equals_reference_nanoflann(oracle):
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref not built (no /root/reference and no prebuilt .so)")
+def test_restatement_equals_reference_nanoflann(oracle, golden_dir):
     sc, (s, d) = _edge_inputs(20000, 32)
+    g = np.load(f"{golden_dir}/ref_pins.npz")
+    for name in ("poses_init", "poses_gt"):   # the reference's answers, stored (tests/golden/make_golden.py:ref_pins)
+        poses = sc[name]
+        a = oracle.KdIndex(sc["pts"][d], "kd").closest_points(sc["pts"][s], poses[s], poses[d], threads=4)
+        assert hashlib.sha256(a[1].tobytes()).hexdigest() == str(g[f"corr_{name}_d2_sha256"])   # minimal squared distance: bit-exact
+        assert np.array_equal(a[0], g[f"corr_{name}_idx"])                                   # no exact ties on jittered data
+    if oracle.ref_lib() is None:
+        return
     ties = 0
     for poses in (sc["poses_init"], sc["poses_gt"]):
         a = oracle.KdIndex(sc["pts"][d], "kd").closest_points(sc["pts"][s], poses[s], poses[d], threads=4)
@@ -91,15 +99,19 @@ def test_pose_graph_knn_is_the_ring(oracle):
 def test_knn_restatement_equals_reference_nanoflann(oracle, golden_dir):
     """Frame::getNeighbours (frame.cpp:208-242): the oracle's k-NN against the reference's nanoflann knnSearch on the
     reference's own scan.  Squared distances must agree bit for bit; indices may differ only inside groups of exactly
-    equal distance (the scan's coordinates are quantised, so such ties exist; nanoflann orders them by traversal)."""
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref not built")
+    equal distance (the scan's coordinates are quantised, so such ties exist; nanoflann orders them by traversal).  The
+    reference's answers are stored (tests/golden/make_golden.py:ref_pins); the library is asked as well when oracle/_ref was built."""
     g = np.load(f"{golden_dir}/bunny_pair.npz")
     pts = g["pts0"]
-    kd = oracle.KdIndex(pts, "kd"); rf = oracle.KdIndex(pts, "ref")
+    pins = np.load(f"{golden_dir}/ref_pins.npz")
+    assert np.array_equal(pins["knn_query"], np.arange(0, len(pts), 53))
+    kd = oracle.KdIndex(pts, "kd"); rf = oracle.KdIndex(pts, "ref") if oracle.ref_lib() is not None else None
     differing = 0
-    for i in range(0, len(pts), 53):
-        a = oracle.knn(kd, pts[i], 10); b = oracle.knn(rf, pts[i], 10)
+    for k, i in enumerate(pins["knn_query"]):
+        a = oracle.knn(kd, pts[i], 10); b = (pins["knn_idx"][k], pins["knn_d2"][k])
+        if rf is not None:
+            live = oracle.knn(rf, pts[i], 10)
+            assert np.array_equal(live[0], b[0]) and np.array_equal(live[1].view(np.uint64), b[1].view(np.uint64))
         assert np.array_equal(a[1].view(np.uint64), b[1].view(np.uint64))
         assert a[0][0] == i == b[0][0] and a[1][0] == 0.0            # the point itself comes first
         if not np.array_equal(a[0], b[0]):

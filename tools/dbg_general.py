@@ -1,9 +1,10 @@
-import numpy as np, sys
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tests')
+import numpy as np, os, sys
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 from oracle import oracle as O
 import mv_lm_icp_b200 as mv
 from mv_lm_icp_b200.api import default_options
-g = np.load('/root/repo/tests/golden/bunny_pair.npz')
+g = np.load(os.path.join(ROOT, 'tests', 'golden', 'bunny_pair.npz'))
 pts = [g["pts0"], g["pts1"], g["pts0"][::2].copy()]; nor = [g["nor0"], g["nor1"], g["nor0"][::2].copy()]
 bump = np.eye(4); bump[:3, :3] = np.array([[1, -0.004, 0.003], [0.004, 1, -0.002], [-0.003, 0.002, 1]]); bump[:3, 3] = [0.002, -0.001, 0.0015]
 poses0 = np.stack([g["pose0"], g["pose1"], bump @ g["pose0"]])

@@ -1,8 +1,9 @@
-import numpy as np, sys
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tests')
+import numpy as np, os, sys
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 from oracle import oracle as O
 import mv_lm_icp_b200 as mv
-g = np.load('/root/repo/tests/golden/bunny_pair.npz')
+g = np.load(os.path.join(ROOT, 'tests', 'golden', 'bunny_pair.npz'))
 pts = [g["pts0"], g["pts1"]]
 eng = mv.Engine(); eng.set_frames(pts, [g["nor0"], g["nor1"]])
 nor, ms = eng.recompute_normals(10)

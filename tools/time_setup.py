@@ -1,10 +1,10 @@
-import sys, time, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, time, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 torch.cuda.init(); torch.zeros(1, device='cuda'); torch.cuda.synchronize()
 import mv_lm_icp_b200 as mv
 from mv_lm_icp_b200 import synth
-sys.path.insert(0, '/root/repo'); import bench
+import bench
 sc = bench.load_scene(3, 20, 200000)
 for rep in range(3):
     t0 = time.perf_counter(); eng = mv.Engine(); t1 = time.perf_counter()
