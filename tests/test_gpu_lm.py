@@ -74,9 +74,10 @@ def test_pipeline_round_matches_oracle(oracle):
 
 @pytest.mark.parametrize("n_views", [29, 40])
 def test_many_views_factor_in_global_memory(oracle, n_views):
-    """The reference's default is --limit=40 frames (main_multiview.cpp:34): 6 x 39 = 234 unknowns, whose Cholesky factor no
-    longer fits the 227 KB of shared memory (n <= 166), so lm_step_kernel keeps it in global memory; 29 views = 168 is the
-    first size on that path.  Same parity bar as the small cases, two consecutive rounds."""
+    """The reference's default is --limit=40 frames (main_multiview.cpp:34): 6 x 39 = 234 unknowns, whose dense Cholesky factor
+    would not fit the 227 KB of shared memory (n <= 166).  The factor is stored as a skyline, and on this ring graph it is a narrow
+    band that stays in shared memory at 29 and 40 views; test_gpu_solver_edges.py::test_factor_crosses_shared_memory_limit runs a
+    graph whose factor moves to global memory and back.  Same parity bar as the small cases, two consecutive rounds."""
     sc = scene(n_views, 1500, 41)
     edges = synth.ring_edges(n_views, 2)
     eng = Engine(); eng.set_frames(sc["pts"], sc["nor"]); eng.set_graph(edges)

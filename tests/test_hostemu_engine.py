@@ -98,6 +98,27 @@ def test_lm_many_views_global_factor(emu, oracle, n_views):
     T.test_many_views_factor_in_global_memory(oracle, n_views)
 
 
+def test_solver_edges(emu, oracle, golden_dir):
+    """tests/test_gpu_solver_edges.py at small sizes: fixed frames anywhere, the factor crossing the shared-memory limit, every
+    option set and termination, a weight-0 robust edge, knn_self / normals at every k, fixed flags toggled in certified rounds."""
+    import test_gpu_solver_edges as T
+    first = emu.order == "ascending"
+    for mask in T.MASKS:
+        for param, cost in (((0, 0), (1, 2), (2, 1)) if first else ((2, 2),)):
+            T.check_fixed_frames(oracle, mask, param, cost, n_points=1000)
+    for name, *_ in T.OPTION_SETS:
+        for param in ((0, 2) if first else (2,)):
+            T.check_option_set(oracle, name, param, n_points=1500)
+    T.check_options_general_path(oracle, golden_dir)
+    T.check_weight0_pipeline(oracle, n_points=1500)
+    for f32 in (True, False):
+        T.check_knn_self(f32, big=3001 if first else 0, sample=100)
+    T.check_normals_every_k(oracle, n_points=2000)
+    T.check_fixed_toggle_in_converged_rounds(oracle, n_views=5, n_points=2003, warm=6)
+    if first:
+        T.check_factor_crosses_shared_memory(oracle, n_points=300)
+
+
 def test_normals(emu, oracle, golden_dir):
     import test_gpu_normals as T
     T.test_normals_match_oracle_synthetic(oracle)
